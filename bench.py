@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- Cassie env-steps/s for the cassie_sim_step_pd hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl reference] [--envs E] [--no-extra]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl reference] [--envs E] [--no-extra] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one control tick (one cassie_sim_step_pd: 0.5 ms of simulated time, 1 physics sub-step) for EVERY environment of the batch.
@@ -13,12 +13,15 @@ Workloads (SURVEY.md section 8d, per GPU; N > 1 = the same workload on every GPU
               left / right phase offset pi, Philox seed 99 (evaluated in the kernel: cassie_batch_set_pd_gait)
 
 value     kernel-only throughput in SINGLE-TICK launches (one cassie_sim_step_pd per launch, the reference's contract): PD rows and state resident
-          in HBM, inputs larger than L2 (independent copies of the batch stepped round-robin, > 1.5 x L2 in total).  The K steps are timed as one
-          block with CUDA events on the launching stream; the block is repeated until the timed total is >= 100 ms and the MEDIAN block is
-          reported (spread beside it); max over ranks.  multi_tick_launches: the same in launches of T <= 50 ticks (PD rows held).
+          in HBM, inputs larger than L2 (independent copies of the batch stepped round-robin, > 1.5 x L2 in total).  Exactly K steps are timed,
+          as one block with CUDA events on the launching stream; max over ranks.  multi_tick_launches: the same K ticks in launches of T <= 50
+          ticks (PD rows held).
 e2e       the same metric through the reference-shaped C-ABI call cassie_sim_step_pd_batch(envs, pd_in_t[] host, state_out_t[] host) with the
           WHOLE state_out_t filled as the reference's state_output_step fills it (the estimator runs inside the kernel): host->device copy of
-          every env's PD input and device->host read of every env's observation inside the timed region.
+          every env's PD input and device->host read of every env's observation inside the timed region, K steps.
+--dump-outputs DIR: after the timed steps, what the last timed step computed, as a caller of the path reads it back (qpos, qvel, time and the
+          observation rows of the batch copy that step advanced; rank 0), is written to DIR/<name>.npy in float64.  Inputs are seeded, so two
+          builds run with the same arguments can be compared output for output.
 roofline  dominant kernel (cassie_step_kernel<float>): HBM figure by the contract's rules (algorithmic state bytes per launch / launch time) and,
           because the kernel is issue / latency bound by design, the issue-slot fraction next to it.
 cpu_baseline / --impl reference: the CPU restatement in oracle/ (physics restated from MuJoCo 2.1.0 semantics + the reference's real closed
@@ -361,36 +364,31 @@ def gpu_arm(args, rank, local_rank, world):
         for bk in copies:
             bk.step(1)
     torch.cuda.synchronize()
-    # how long is one tick, roughly -> how many K-step blocks make >= 100 ms
-    p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    p0.record()
-    for i in range(8):
-        copies[i % nb_copies].step(1)
-    p1.record(); torch.cuda.synchronize()
-    est_ms = max(1e-3, p0.elapsed_time(p1) / 8)
-    nblocks = max(3, int(math.ceil(MIN_TIMED_MS / (est_ms * K))))
     launches0 = sum(bk.launch_count() for bk in copies)
     sampler = ClockSampler(local_rank) if rank == 0 else None
 
-    def run_blocks(ticks_per_launch):
-        """nblocks blocks of exactly K steps; each block bracketed by events on the launching stream; returns per-block ms"""
-        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(nblocks)]
-        i = 0
+    def run_block(ticks_per_launch):
+        """exactly K steps, bracketed by events on the launching stream; returns (ms, the copy the last launch advanced)"""
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
-        for e0, e1 in ev:
-            e0.record()
-            for _ in range(K // ticks_per_launch):
-                if ticks_per_launch == 1:
-                    W.before_step(copies[i % nb_copies], i % nb_copies, nb_copies)
-                copies[i % nb_copies].step(ticks_per_launch); i += 1
-            e1.record()
+        torch.cuda._sleep(2_000_000)   # ~1 ms device-side wait: the first launches queue up behind it, so the window holds no host enqueue gap
+        e0.record()
+        for i in range(K // ticks_per_launch):
+            if ticks_per_launch == 1:
+                W.before_step(copies[i % nb_copies], i % nb_copies, nb_copies)
+            copies[i % nb_copies].step(ticks_per_launch)
+        e1.record()
         barrier()
-        return [e0.elapsed_time(e1) for e0, e1 in ev]
+        return e0.elapsed_time(e1), copies[(K // ticks_per_launch - 1) % nb_copies]
 
-    blk = run_blocks(1)                                  # headline: single-tick launches
+    med, last = run_block(1)                             # headline: single-tick launches
     launches = sum(bk.launch_count() for bk in copies) - launches0
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in (('qpos', last.qpos()), ('qvel', last.qvel()), ('time', last.time()), ('obs', last.obs())):
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), np.ascontiguousarray(arr, dtype=np.float64))
     T = max(t for t in range(1, 51) if K % t == 0)       # multi-tick launches of T ticks, PD rows held
-    blk_multi = run_blocks(T) if T > 1 else blk
+    med_multi = run_block(T)[0] if T > 1 else med
     # ---- one copy, 256 MiB memset between launches (the other flush method; per-launch events; reported beside the value)
     nfl = min(K, 50)
     evf = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(nfl)]
@@ -411,13 +409,9 @@ def gpu_arm(args, rank, local_rank, world):
     out = (P.state_out_t * n)()
 
     def time_e2e():
-        for _ in range(3):
+        for _ in range(4):
             b.L.cassie_sim_step_pd_batch(b.h, C.byref(pd), C.byref(out))
-        barrier()
-        t0 = time.perf_counter()
-        b.L.cassie_sim_step_pd_batch(b.h, C.byref(pd), C.byref(out))
-        one = time.perf_counter() - t0
-        steps = max(10, K, int(math.ceil(MIN_TIMED_MS * 1e-3 / max(one, 1e-6))))
+        steps = K
         tm = (C.c_double * 6)()
         b.L.cassie_batch_aos_timing(b.h, tm, 1)
         barrier()
@@ -495,7 +489,6 @@ def gpu_arm(args, rank, local_rank, world):
             except Exception as ex:
                 others['config%d' % c] = {'error': repr(ex)}
     # ---- reduce over ranks: a rank's figure is its median block; the job's is the slowest rank's
-    med, med_multi = float(np.median(blk)), float(np.median(blk_multi))
     t = torch.tensor([med, med_multi, t_e2e / e2e_steps, t_e2e_off / e2e_steps_off, ms_flush], dtype=torch.float64, device='cuda')
     per_rank = None
     if dist:
@@ -525,9 +518,8 @@ def gpu_arm(args, rank, local_rank, world):
                 'config': {'workload': cfg['name'], 'envs_per_gpu': n, 'ticks_per_step': 1, 'ticks_per_launch': 1, 'parallelism': 'env-sharded x%d (no data-path collective)' % world,
                            'l2': 'inputs larger than L2: %d independent copies of the batch (%.0f MB) stepped round-robin' % (nb_copies, nb_copies * per_copy / 1e6),
                            'model': 'compiled table of model/%s.xml' % cfg['model']},
-                'timing': {'blocks': nblocks, 'steps_per_block': K, 'block_ms_median': med, 'block_ms_min': float(min(blk)), 'block_ms_max': float(max(blk)),
-                           'spread': (float(max(blk)) - float(min(blk))) / med, 'timed_ms_total': float(sum(blk)),
-                           'note': 'each block = exactly K single-tick launches between two CUDA events on the launching stream; median block reported, max over ranks'},
+                'timing': {'blocks': 1, 'steps_per_block': K, 'timed_ms_total': med,
+                           'note': 'exactly K single-tick launches between two CUDA events on the launching stream; max over ranks'},
                 'multi_tick_launches': {'ticks_per_launch': T, 'ms_per_step': med_multi / K, 'env_steps_per_s': world * n * K / (med_multi * 1e-3),
                                         'note': 'cassie_batch_step(b, T): T control ticks per launch with the PD rows held, no host round trip; same blocks'},
                 'l2_memset_flush_mode': {'ms_per_step': ms_flush, 'env_steps_per_s_this_rank': n / (ms_flush * 1e-3), 'note': 'one copy, 256 MiB memset between launches, per-launch events'},
@@ -559,6 +551,7 @@ def main():
     ap.add_argument('--config', type=int, default=2, choices=sorted(CONFIGS))
     ap.add_argument('--envs', type=int, default=0, help='environments per GPU (default: the configuration\'s own size)')
     ap.add_argument('--no-extra', dest='no_extra', action='store_true', help='skip the short runs of BASELINE configs 3-5 beside the config-2 line')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy')
     args = ap.parse_args()
     rank, local_rank, world = int(os.environ.get('RANK', 0)), int(os.environ.get('LOCAL_RANK', 0)), int(os.environ.get('WORLD_SIZE', 1))
     if args.warmup < 3:

@@ -77,6 +77,18 @@ void probe_core(const double *in, const double *u, double ch8, double *out) {
   cassie_core_sim_free(c);
 }
 
+/* the chain oracle/fuzz_agility.c checks, on fresh blocks: in[45] (cassie_out), a whole pd_in_t, radio channel 8 -> pd[10] = cassie_user_in_t.torque
+ * of pd_input_step, core[10] = the drive torques cassie_core_sim_step makes of them */
+void probe_pd_core(const double *in, const pd_in_t *u, double ch8, double *pd, double *core) {
+  cassie_out_t o; fill(&o, in); o.pelvis.radio.channel[8] = ch8;
+  cassie_user_in_t ui; memset(&ui, 0, sizeof ui);
+  pd_input_t *p = pd_input_alloc(); pd_input_setup(p); pd_input_step(p, u, &o, &ui); pd_input_free(p);
+  for (int i = 0; i < 10; i++) pd[i] = ui.torque[i];
+  cassie_in_t ci; memset(&ci, 0, sizeof ci);
+  cassie_core_sim_t *c = cassie_core_sim_alloc(); cassie_core_sim_setup(c); cassie_core_sim_step(c, &ui, &o, &ci); cassie_core_sim_free(c);
+  for (int i = 0; i < 10; i++) { const cassie_leg_in_t *l = i < 5 ? &ci.leftLeg : &ci.rightLeg; const elmo_in_t *t[5] = {&l->hipRollDrive, &l->hipYawDrive, &l->hipPitchDrive, &l->kneeDrive, &l->footDrive}; core[i] = t[i % 5]->torque; }
+}
+
 /* as probe_est, plus the drives' measured torques: in[45..54] */
 void probe_est_tq(const double *in, int ncalls, double *out) {
   cassie_out_t o; state_out_t y; fill(&o, in);

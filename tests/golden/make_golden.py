@@ -8,6 +8,9 @@ Runs ONLY in the build container (needs /root/reference); the GPU box uses the c
              initial state (free fall, touch-down, load transfer): its stateless outputs that feed its filters, and the filters' outputs
   agility_vectors.npz   input/output pairs of the reference's closed Agility blocks (pd_input_step incl. taskPd, cassie_core_sim_step,
              state_output_step from src/libagilitycassie.a via oracle/_ref/liboracle_ref.so; layout: oracle/probe_estimator.c)
+  reference_bus_layout.json   the reference's bus struct layout (field lists of its ctypes mirror, gcc offsets from its headers)
+  archive_runs.npz   the same blocks in closed loops of the oracle's simulator (sampled records), on the fuzz inputs of oracle/fuzz_agility.c's
+             kind and on random estimator inputs: what the twin, controller and estimator tests compare against (archive_runs below)
 """
 import os
 import sys
@@ -89,9 +92,88 @@ def estimator_sequence(T=400):
     print('wrote estimator_sequence.npz', T)
 
 
+def archive_runs(every=50, n_fuzz=100, n_random=150):
+    """what tests/test_agility_twins.py, tests/test_estimator_filter.py and the GPU estimator tests compare against, from the REAL closed blocks
+    (oracle/_ref/liboracle_ref.so):
+      <run>_tick / _cassie_out / _state_out / _qpos   closed loops of the oracle's simulator with the real blocks, sampled every `every` ticks:
+             the cassie_out_t record and the state_out_t the block made of it (raw struct bytes) and qpos.  Runs: 'pd' = the fixed motor-PD
+             controller from the initial state (1200 ticks), 'zero' = zero pd_in_t (1000 ticks), 'spin' = the fixed PD from a spinning attitude
+             stored with w < 0 (700 ticks)
+      fuzz<mode>_pd / _core   pd_input_step and cassie_core_sim_step on the first n_fuzz inputs of test_agility_twins.fuzz_inputs(mode)
+      est_random_feet   the foot outputs (state_out_t flattened [22:35] and [41:54]) on the first n_random inputs of test_agility_twins.random_foot_inputs()
+      est_kinematics_feet   the foot positions ([22:25] and [41:44]) on the inputs of test_agility_twins.kinematics_inputs()"""
+    import ctypes as C
+    import importlib
+    import numpy as np
+    sys.path.insert(0, REPO)
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    import oracle as O
+    import test_agility_twins as T
+    from conftest import PD_DGAIN, PD_PGAIN, PD_TARGET
+    pkg = importlib.import_module('cassie-mujoco-sim_b200')
+    O.build(ref=True)
+    out = {}
+    fixed = O.make_pd(pTarget=PD_TARGET, pGain=PD_PGAIN, dGain=PD_DGAIN)
+    for name, u, spin, ticks in (('pd', fixed, False, 1200), ('zero', O.make_pd(), False, 1000), ('spin', fixed, True, 700)):
+        o = O.OracleSim(os.path.join(HERE, 'cassie.omodel'), ref=True)
+        if spin:
+            T.spin_setup(o)
+        y, co = pkg.state_out_t(), (C.c_char * 1336)()
+        rows = []
+        for k in range(ticks):
+            o.step_pd(u, y, co)
+            if (k + 1) % every == 0:
+                rows.append((k, np.frombuffer(bytes(co), np.uint8), np.frombuffer(bytes(y), np.uint8), o.arr('qpos').copy()))
+        for i, key in enumerate(('tick', 'cassie_out', 'state_out', 'qpos')):
+            out[name + '_' + key] = np.array([r[i] for r in rows])
+    L = O.load(ref=True)
+    dp = C.POINTER(C.c_double)
+    L.probe_pd_core.argtypes = [dp, C.c_void_p, C.c_double, dp, dp]
+    L.probe_est.argtypes = [dp, C.c_int, dp]
+    for mode in (0, 1):
+        pd, core = np.zeros((n_fuzz, 10)), np.zeros((n_fuzz, 10))
+        for i, (x, ch8, u) in enumerate(T.fuzz_inputs(mode, n_fuzz, pkg)):
+            L.probe_pd_core(x.ctypes.data_as(dp), C.byref(u), ch8, pd[i].ctypes.data_as(dp), core[i].ctypes.data_as(dp))
+        out['fuzz%d_pd' % mode], out['fuzz%d_core' % mode] = pd, core
+
+    def est(x):
+        e = np.zeros(123)
+        L.probe_est(np.ascontiguousarray(x).ctypes.data_as(dp), 1, e.ctypes.data_as(dp))
+        return e
+    out['est_random_feet'] = np.array([np.concatenate([e[22:35], e[41:54]]) for e in map(est, T.random_foot_inputs(n_random))])
+    out['est_kinematics_feet'] = np.array([np.concatenate([e[22:25], e[41:44]]) for e in map(est, (x for x, _ in T.kinematics_inputs()))])
+    np.savez_compressed(os.path.join(HERE, 'archive_runs.npz'), **out)
+    print('wrote archive_runs.npz', {k: v.shape for k, v in out.items()})
+
+
+def bus_layout():
+    """reference_bus_layout.json: the bus structs' field lists in the reference's generated ctypes mirror (example/cassiemujoco_ctypes.py) and
+    the sizes / offsets gcc gives them from the reference's headers (the probes of tests/test_abi.py)"""
+    import json
+    import pathlib
+    import re
+    import tempfile
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    import test_abi
+    txt = open(os.path.join(REF, 'example', 'cassiemujoco_ctypes.py')).read()
+    fields = {}
+    for struct in ('struct_c__SA_pd_in_t', 'struct_c__SA_state_out_t', 'struct_c__SA_state_pelvis_out_t'):
+        m = re.search(struct + r'\._fields_ = \[(.*?)\]\n', txt, flags=re.S) or re.search(r'class ' + struct + r'\(.*?_fields_ = \[(.*?)\]\n', txt, flags=re.S)
+        fields[struct] = [f for f in re.findall(r"\('(\w+)'", m.group(1)) if not f.startswith('PADDING')]
+    with tempfile.TemporaryDirectory() as d:
+        offsets = test_abi.bus_offsets(pathlib.Path(d), 'ref', ['pd_in_t.h', 'state_out_t.h', 'cassie_out_t.h', 'cassie_in_t.h', 'cassie_user_in_t.h'],
+                                       os.path.join(REF, 'include'))
+    with open(os.path.join(HERE, 'reference_bus_layout.json'), 'w') as f:
+        json.dump({'ctypes_fields': fields, 'offsets': offsets}, f, indent=1)
+        f.write('\n')
+    print('wrote reference_bus_layout.json')
+
+
 def main():
+    bus_layout()
     agility_vectors()
     estimator_sequence()
+    archive_runs()
     for name in MODELS:
         m = mc.compile_mjcf(os.path.join(REF, 'model', name + '.xml'))
         mc.write_omodel(m, os.path.join(HERE, name + '.omodel'))

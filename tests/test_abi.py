@@ -1,13 +1,14 @@
 """C-ABI checks that need no GPU: the library loads, exports every symbol include/cassie_b200.h declares, the bus structs have
 the reference's sizes, and the product fails loudly (no CPU fallback) when no CUDA device is visible."""
 import ctypes as C
+import json
 import os
 import re
 import sys
 
 import pytest
 
-from conftest import REFERENCE, REPO, have_reference, product
+from conftest import GOLDEN, REFERENCE, REPO, have_reference, product
 
 
 def declared_functions():
@@ -27,17 +28,11 @@ def test_library_exports_every_declared_symbol(pkg):
 
 def test_bus_struct_sizes_match_reference_ctypes(pkg):
     assert C.sizeof(pkg.pd_in_t) == 952 and C.sizeof(pkg.state_out_t) == 992
-    if not have_reference():
-        pytest.skip('reference checkout not present')
-    # the reference's generated ctypes mirror cannot be imported (it dlopens libcassiemujoco.so at import), so read its struct sizes
-    # the same way clang2py recorded them: field lists.  Compare field names and order instead.
-    txt = open(os.path.join(REFERENCE, 'example', 'cassiemujoco_ctypes.py')).read()
+    # the reference's generated ctypes mirror (example/cassiemujoco_ctypes.py) records the field lists clang2py saw; they are committed in
+    # tests/golden/reference_bus_layout.json.  Compare field names and order.
+    ref = json.load(open(os.path.join(GOLDEN, 'reference_bus_layout.json')))['ctypes_fields']
     for struct, mine in (('struct_c__SA_pd_in_t', pkg.pd_in_t), ('struct_c__SA_state_out_t', pkg.state_out_t), ('struct_c__SA_state_pelvis_out_t', pkg.state_pelvis_out_t)):
-        m = re.search(struct + r'\._fields_ = \[(.*?)\]\n', txt, flags=re.S) or re.search(r'class ' + struct + r'\(.*?_fields_ = \[(.*?)\]\n', txt, flags=re.S)
-        assert m, struct
-        ref_fields = re.findall(r"\('(\w+)'", m.group(1))
-        ref_fields = [f for f in ref_fields if not f.startswith('PADDING')]
-        assert ref_fields == [f[0] for f in mine._fields_], struct
+        assert ref[struct] == [f[0] for f in mine._fields_], struct
 
 
 def test_no_gpu_means_loud_failure_not_fallback(pkg):
@@ -94,12 +89,7 @@ def test_c_example_builds_against_the_header_and_fails_loudly_without_a_gpu(pkg,
     assert r.returncode == 1 and 'no CUDA device' in r.stderr, (r.returncode, r.stderr)
 
 
-def test_bus_struct_offsets_equal_the_reference_headers(tmp_path):
-    """field offsets of every bus struct: include/cassie_bus.h against the reference's own headers, both compiled by gcc (two programs, same probes)"""
-    import subprocess
-    if not have_reference():
-        pytest.skip('reference checkout not present')
-    probes = r'''
+BUS_PROBES = r'''
 #include <stdio.h>
 #include <stddef.h>
 #define P(T, f) printf(#T "." #f " %zu\n", offsetof(T, f))
@@ -114,15 +104,24 @@ int main(void) {
   return 0;
 }
 '''
-    outs = []
-    for tag, hdrs, inc in (('mine', ['cassie_bus.h'], os.path.join(REPO, 'include')),
-                           ('ref', ['pd_in_t.h', 'state_out_t.h', 'cassie_out_t.h', 'cassie_in_t.h', 'cassie_user_in_t.h'], os.path.join(REFERENCE, 'include'))):
-        src = tmp_path / (tag + '.c')
-        src.write_text('#include <stdbool.h>\n' + ''.join('#include "%s"\n' % h for h in hdrs) + probes)
-        exe = str(tmp_path / tag)
-        subprocess.check_call(['gcc', '-std=c11', '-I', inc, str(src), '-o', exe])
-        outs.append(subprocess.check_output([exe], text=True))
-    assert outs[0] == outs[1] and 'sizes 952 992 1336' in outs[0], outs
+
+
+def bus_offsets(tmp_path, tag, hdrs, inc):
+    """sizes and field offsets of the bus structs as gcc lays them out from the headers `hdrs` under `inc`"""
+    import subprocess
+    src = tmp_path / (tag + '.c')
+    src.write_text('#include <stdbool.h>\n' + ''.join('#include "%s"\n' % h for h in hdrs) + BUS_PROBES)
+    exe = str(tmp_path / tag)
+    subprocess.check_call(['gcc', '-std=c11', '-I', inc, str(src), '-o', exe])
+    return subprocess.check_output([exe], text=True)
+
+
+def test_bus_struct_offsets_equal_the_reference_headers(tmp_path):
+    """field offsets of every bus struct: include/cassie_bus.h compiled by gcc against the same probes compiled on the reference's own headers
+    (their output is committed in tests/golden/reference_bus_layout.json)"""
+    mine = bus_offsets(tmp_path, 'mine', ['cassie_bus.h'], os.path.join(REPO, 'include'))
+    ref = json.load(open(os.path.join(GOLDEN, 'reference_bus_layout.json')))['offsets']
+    assert mine == ref and 'sizes 952 992 1336' in mine, (mine, ref)
 
 
 def test_every_name_the_reference_binding_resolves_is_exported(tmp_path):

@@ -1,54 +1,85 @@
 """The closed Agility blocks (pd_input_step motor branch, cassie_core_sim_step): twins vs the reference's archive."""
 import os
-import re
-import subprocess
 
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, PD_DGAIN, PD_PGAIN, PD_TARGET, REFERENCE, REPO
+from conftest import GOLDEN, PD_DGAIN, PD_PGAIN, PD_TARGET, REPO
 
-FUZZ = os.path.join(REPO, 'oracle', '_ref', 'fuzz_agility')
-ARCHIVE = os.path.join(REFERENCE, 'src', 'libagilitycassie.a')
+ARCHIVE_RUNS = os.path.join(GOLDEN, 'archive_runs.npz')   # outputs of the REAL closed blocks (tests/golden/make_golden.py archive_runs)
 
 
-def _fuzz_binary():
-    if os.path.exists(ARCHIVE):
-        subprocess.check_call(['make', '-s', '-C', os.path.join(REPO, 'oracle'), 'fuzz', 'ref'])
-    if not os.path.exists(FUZZ):
-        pytest.skip('neither the reference archive nor a prebuilt oracle/_ref is available')
-    return FUZZ
+def archive_runs():
+    return np.load(ARCHIVE_RUNS)
+
+
+def fuzz_inputs(mode, n, pkg, seed=12345):
+    """the inputs oracle/fuzz_agility.c draws: drive angles inside the joint ranges (mode 0: mostly well inside, a quarter of them anywhere in
+    range; mode 1: anywhere), radio channel 8 random on every 17th input, random motor PD and, on two thirds of the inputs, random task PD.
+    Yields (cassie_out as the 45 numbers of oracle/probe_estimator.c, radio channel 8, pd_in_t)."""
+    rng = np.random.default_rng(seed + mode)
+    lo, hi = np.array([-0.3, -0.4, -0.9, -2.9, -2.5] * 2), np.array([0.3, 0.4, 1.4, -0.6, -0.5] * 2)
+    for it in range(n):
+        x = np.zeros(45)
+        x[32] = 1
+        w = np.where((mode == 1) | (rng.random(10) < 0.25), 1.0, 0.55)
+        x[0:10] = 0.5 * (lo + hi) + 0.5 * (hi - lo) * w * rng.uniform(-1, 1, 10)
+        x[5] = -x[5]
+        x[10:20] = rng.uniform(-8, 8, 10)
+        x[20:26] = rng.uniform([-0.2, 0.8, -2.4] * 2, [0.2, 2.6, -0.6] * 2)
+        x[26:32] = rng.uniform(-6, 6, 6)
+        ch8 = rng.uniform(-1, 1) if it % 17 == 0 else 1.0
+        u = pkg.pd_in_t()
+        for sd, leg in enumerate((u.leftLeg, u.rightLeg)):
+            m = rng.uniform([-50, -2, -3, 0, 0], [50, 2, 3, 200, 10], (5, 5))
+            for k in range(5):
+                leg.motorPd.torque[k], leg.motorPd.pTarget[k], leg.motorPd.dTarget[k], leg.motorPd.pGain[k], leg.motorPd.dGain[k] = m[k]
+            if it % 3:
+                t = rng.uniform([-30, -1, -2, 0, 0], [30, 1, 2, 300, 10], (6, 5)) * (rng.random((6, 5)) < [1, 1, 1, 0.75, 0.75])
+                for k in range(6):
+                    leg.taskPd.torque[k], leg.taskPd.pTarget[k], leg.taskPd.dTarget[k], leg.taskPd.pGain[k], leg.taskPd.dGain[k] = t[k]
+        yield x, ch8, u
 
 
 @pytest.mark.parametrize('mode', [0, 1])
-def test_oracle_twins_match_archive_on_fuzz(mode):
-    out = subprocess.check_output([_fuzz_binary(), '100000', str(mode)], text=True)
-    m = re.search(r'pd twin - archive\| = ([0-9.e+-]+)\s+max\|core twin - archive\| = ([0-9.e+-]+)', out)
-    assert m, out
-    assert float(m.group(1)) <= 1e-9 and float(m.group(2)) <= 1e-9, out   # torques up to ~1e4 N m with the fuzzed task gains
+def test_oracle_twins_match_archive_on_fuzz(mode, oracle_mod, pkg):
+    import ctypes as C
+    V = archive_runs()
+    L = oracle_mod.load()
+    dp = C.POINTER(C.c_double)
+    L.osim_fill_cassie_out.argtypes = [C.c_void_p, dp]
+    L.o_pd_input_step.argtypes = [C.c_void_p, C.c_void_p, dp]
+    L.o_core_sim_step.argtypes = [dp, C.c_void_p, dp]
+    want_pd, want_core = V['fuzz%d_pd' % mode], V['fuzz%d_core' % mode]
+    err_pd, err_core = 0.0, 0.0
+    for (x, ch8, u), pdq, core in zip(fuzz_inputs(mode, len(want_pd), pkg), want_pd, want_core):
+        co = (C.c_char * 1336)()
+        L.osim_fill_cassie_out(co, np.ascontiguousarray(x).ctypes.data_as(dp))
+        L.osim_set_radio8(co, C.c_double(ch8))
+        tq, out = (C.c_double * 10)(), (C.c_double * 10)()
+        L.o_pd_input_step(C.byref(u), co, tq)
+        L.o_core_sim_step(np.ascontiguousarray(pdq).ctypes.data_as(dp), co, out)    # fed the archive's own pd_input_step output, as the fuzz does
+        err_pd, err_core = max(err_pd, np.abs(np.array(tq[:]) - pdq).max()), max(err_core, np.abs(np.array(out[:]) - core).max())
+    assert len(want_pd) >= 100 and np.abs(want_core).max() > 100
+    assert err_pd <= 1e-9 and err_core <= 1e-9, (err_pd, err_core)   # torques up to ~1e4 N m with the fuzzed task gains
 
 
 def test_product_controller_matches_archive_in_closed_loop(oracle_mod):
     """the product's controller stage (step_core.inl, run through the host emulation in fp64) against the oracle linked with the
     REAL archive blocks, over BASELINE config 1 (zero pd_in_t, 1000 ticks: the collapsing robot drives joints into the safety
-    layer's soft limits) and the fixed-PD controller"""
-    import oracle as O
-    _fuzz_binary()
-    if not os.path.exists(O.lib_path(ref=True)):
-        pytest.skip('oracle/_ref/liboracle_ref.so not available')
+    layer's soft limits) and the fixed-PD controller; the archive's trajectory is stored every 50 ticks"""
     import emu_harness as E
-    for u, pd in ((O.make_pd(), np.zeros(50)),
-                  (O.make_pd(pTarget=PD_TARGET, pGain=PD_PGAIN, dGain=PD_DGAIN), np.concatenate([np.zeros(10), PD_TARGET, np.zeros(10), PD_PGAIN, PD_DGAIN]))):
-        o = O.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'), ref=True)
+    V = archive_runs()
+    for run, pd in (('zero', np.zeros(50)), ('pd', np.concatenate([np.zeros(10), PD_TARGET, np.zeros(10), PD_PGAIN, PD_DGAIN]))):
         e = E.EmuSim(os.path.join(REPO, 'cassie-mujoco-sim_b200', 'models', 'cassie.cmodel'))
+        ticks, want = list(V[run + '_tick']), V[run + '_qpos']
         worst, safety = 0.0, 0
-        for k in range(1000):
-            o.step_pd(u)
+        for k in range(ticks[-1] + 1):
             e.step(pd)
-            worst = max(worst, np.abs(e.get('qpos')[:35] - o.arr('qpos')).max())
-            knee = o.arr('qpos')[14]
-            safety += knee < -2.5727
-        assert worst < 1e-9, worst
+            safety += e.get('qpos')[14] < -2.5727
+            if k in ticks:
+                worst = max(worst, np.abs(e.get('qpos')[:35] - want[ticks.index(k)]).max())
+        assert worst < 1e-9, (run, worst)
         if not pd.any():
             assert safety > 50     # the safety layer really was exercised
 
@@ -65,99 +96,91 @@ def field(y, path):
     return np.array(y[:])
 
 
+def spin_setup(o):
+    """a spinning attitude stored with w < 0 (the estimator reports the w >= 0 twin)"""
+    o.arr('qpos')[3:7] = [-0.995, 0.02, -0.03, 0.09]
+    o.arr('qvel')[3:6] = [0.5, -0.4, 0.6]
+
+
 def test_estimator_twin_matches_archive_in_closed_loop(oracle_mod, pkg):
     """the decoded stateless subset of state_output_step (oracle o_state_output_step) against the REAL estimator, fed the same cassie_out
-    along a falling-and-catching trajectory (large joint excursions; an IMU quaternion with w < 0)"""
+    along a falling-and-catching trajectory (large joint excursions; an IMU quaternion with w < 0); the archive's records every 50 ticks"""
     import ctypes as C
-    import oracle as O
-    _fuzz_binary()
-    if not os.path.exists(O.lib_path(ref=True)):
-        pytest.skip('oracle/_ref/liboracle_ref.so not available')
-    L = O.load(ref=True)
+    V = archive_runs()
+    L = oracle_mod.load()
     L.o_state_output_step.argtypes = [C.c_void_p, C.c_void_p]
-    L.osim_cassie_out.restype = C.c_void_p
     worst = {k: 0.0 for k in DECODED}
-    for u, setup in ((O.make_pd(), None), (O.make_pd(pTarget=PD_TARGET, pGain=PD_PGAIN, dGain=PD_DGAIN), 'spin')):
-        o = O.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'), ref=True)
-        if setup == 'spin':
-            o.arr('qpos')[3:7] = [-0.995, 0.02, -0.03, 0.09]      # same kind of attitude, stored with w < 0: the estimator reports the w >= 0 twin
-            o.arr('qvel')[3:6] = [0.5, -0.4, 0.6]
-        y, y2, co = pkg.state_out_t(), pkg.state_out_t(), (C.c_char * 1336)()
-        saw_neg = False
-        for k in range(700):
-            o.step_pd(u, y, co)                         # y: real estimator on this tick's cassie_out (copied into co)
-            L.o_state_output_step(C.byref(co), C.byref(y2))
+    for run in ('zero', 'spin'):
+        for co, ya in zip(V[run + '_cassie_out'], V[run + '_state_out']):
+            y, y2 = pkg.state_out_t.from_buffer_copy(ya.tobytes()), pkg.state_out_t()
+            L.o_state_output_step((C.c_char * 1336).from_buffer_copy(co.tobytes()), C.byref(y2))
             for f in DECODED:
                 worst[f] = max(worst[f], np.abs(field(y, f) - field(y2, f)).max())
-            saw_neg |= o.arr('sensordata')[16] < 0
-        if setup == 'spin':
-            assert saw_neg
+    assert V['spin_qpos'][:, 3].min() < 0
     for f, w in worst.items():
         assert w < 1e-11, (f, w)
 
 
-def _probe(O):
-    import ctypes as C
-    _fuzz_binary()
-    if not os.path.exists(O.lib_path(ref=True)):
-        pytest.skip('oracle/_ref/liboracle_ref.so not available')
-    L = O.load(ref=True)
-    L.probe_est.argtypes = [C.POINTER(C.c_double), C.c_int, C.POINTER(C.c_double)]
+def random_foot_inputs(n, seed=11):
+    """arbitrary angles / rates, as the 45 cassie_out numbers of oracle/probe_estimator.c"""
+    rng = np.random.default_rng(seed)
+    for it in range(n):
+        x = np.zeros(45)
+        x[32] = 1
+        x[0:10], x[10:20], x[20:26], x[26:32] = rng.uniform(-3, 3, 10), rng.uniform(-8, 8, 10), rng.uniform(-3, 3, 6), rng.uniform(-8, 8, 6)
+        yield x
 
-    def est(inp):
-        a, out = np.ascontiguousarray(inp, dtype=np.float64), np.zeros(123)
-        L.probe_est(a.ctypes.data_as(C.POINTER(C.c_double)), 1, out.ctypes.data_as(C.POINTER(C.c_double)))
-        return out
-    return est
+
+def kinematics_inputs(n=50, seed=4):
+    """random leg configurations inside the joint ranges: (the 45 cassie_out numbers, qpos of the same configuration)"""
+    rng = np.random.default_rng(seed)
+    lo, hi = np.array([-0.25, -0.35, -0.8, -2.7, -2.4]), np.array([0.3, 0.35, 1.3, -0.7, -0.6])
+    for it in range(n):
+        mL, mR, sh, ta = rng.uniform(lo, hi), rng.uniform(lo, hi), rng.uniform(-0.05, 0.05, 2), rng.uniform(0.9, 2.0, 2)
+        q = np.zeros(35)
+        q[2], q[3], q[10], q[24] = 1.01, 1, 1, 1
+        q[[7, 8, 9, 14, 20]], q[15], q[16] = mL, sh[0], ta[0]
+        q[[21, 22, 23, 28, 34]], q[29], q[30] = mR, sh[1], ta[1]
+        x = np.zeros(45)
+        x[32] = 1
+        x[0:5], x[5:10], x[20], x[21], x[23], x[24] = mL, mR, sh[0], ta[0], sh[1], ta[1]
+        yield x, q
 
 
 def test_estimator_twin_on_random_inputs(oracle_mod):
     """o_est_foot against the archive on arbitrary angles / rates (far outside what a trajectory visits: all mat2quat branches)"""
     import ctypes as C
-    est, L = _probe(oracle_mod), oracle_mod.load()
+    want = archive_runs()['est_random_feet']
+    L = oracle_mod.load()
     L.o_est_foot.argtypes = [C.c_int] + [C.POINTER(C.c_double)] * 6
-    rng, worst = np.random.default_rng(11), 0.0
-    for it in range(2000):
-        x = np.zeros(45)
-        x[32] = 1
-        x[0:10], x[10:20], x[20:26], x[26:32] = rng.uniform(-3, 3, 10), rng.uniform(-8, 8, 10), rng.uniform(-3, 3, 6), rng.uniform(-8, 8, 6)
-        e = est(x)
+    worst = 0.0
+    for x, e in zip(random_foot_inputs(len(want)), want):
         for sd in range(2):
             ang = (C.c_double * 7)(*x[5 * sd:5 * sd + 4], x[20 + 3 * sd], x[21 + 3 * sd], x[5 * sd + 4])
             rate = (C.c_double * 7)(*x[10 + 5 * sd:14 + 5 * sd], x[26 + 3 * sd], x[27 + 3 * sd], x[14 + 5 * sd])
             out = [(C.c_double * n)() for n in (3, 4, 3, 3)]
             L.o_est_foot(sd, ang, rate, *out)
             got = np.concatenate([np.array(a[:]) for a in out])
-            worst = max(worst, np.abs(got - e[22 + 19 * sd:35 + 19 * sd]).max())
-    assert worst < 1e-12, worst
+            worst = max(worst, np.abs(got - e[13 * sd:13 * sd + 13]).max())
+    assert len(want) >= 150 and worst < 1e-12, worst
 
 
 def test_archive_kinematics_pin_the_mjcf_compiler(oracle_mod):
     """an independent check of the model compiler's kinematic tables: the foot point computed by the oracle's mj_kinematics on the compiled
     model/cassie.xml equals the closed estimator's own forward kinematics (which carries Agility's constants) to the MJCF's 5-digit rounding"""
-    est = _probe(oracle_mod)
+    want = archive_runs()['est_kinematics_feet']
     o = oracle_mod.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'))
     names = open(os.path.join(GOLDEN, 'cassie.omodel')).read().split('names_body')[1].split('\n')[0].split()[2:]
     pel, feet = names.index('cassie-pelvis'), (names.index('left-foot'), names.index('right-foot'))
-    rng, worst = np.random.default_rng(4), 0.0
-    lo, hi = np.array([-0.25, -0.35, -0.8, -2.7, -2.4]), np.array([0.3, 0.35, 1.3, -0.7, -0.6])
-    for it in range(50):
-        mL, mR, sh, ta = rng.uniform(lo, hi), rng.uniform(lo, hi), rng.uniform(-0.05, 0.05, 2), rng.uniform(0.9, 2.0, 2)
-        q = o.arr('qpos')
-        q[:] = 0
-        q[2], q[3], q[10], q[24] = 1.01, 1, 1, 1
-        q[[7, 8, 9, 14, 20]], q[15], q[16] = mL, sh[0], ta[0]
-        q[[21, 22, 23, 28, 34]], q[29], q[30] = mR, sh[1], ta[1]
+    worst = 0.0
+    for (x, q), e in zip(kinematics_inputs(), want):
+        o.arr('qpos')[:] = q
         o.forward()
         xp, xm = o.arr('xpos').reshape(-1, 3), o.arr('xmat').reshape(-1, 3, 3)
-        x = np.zeros(45)
-        x[32] = 1
-        x[0:5], x[5:10], x[20], x[21], x[23], x[24] = mL, mR, sh[0], ta[0], sh[1], ta[1]
-        e = est(x)
         for sd, fb in enumerate(feet):
             p = xm[pel].T @ (xp[fb] + xm[fb] @ np.array([0.01762, 0.05219, 0]) - xp[pel])
-            worst = max(worst, np.abs(p - e[22 + 19 * sd:25 + 19 * sd]).max())
-    assert worst < 5e-7, worst
+            worst = max(worst, np.abs(p - e[3 * sd:3 * sd + 3]).max())
+    assert len(want) == 50 and worst < 5e-7, worst
 
 
 def test_twins_against_committed_archive_vectors(oracle_mod, pkg):
@@ -211,7 +234,6 @@ def test_toe_heel_force_twin(oracle_mod, pkg):
     bar is its own rounding noise (a few mN on forces of ~100 N), not 1e-12: |twin - archive| <= 2e-2 N + 2e-4 |F| in closed loop and on the
     committed random vectors whose deflections are physically plausible"""
     import ctypes as C
-    import oracle as O
     V = np.load(os.path.join(GOLDEN, 'agility_vectors.npz'))
     L = oracle_mod.load()
     dp = C.POINTER(C.c_double)
@@ -228,21 +250,17 @@ def test_toe_heel_force_twin(oracle_mod, pkg):
             assert np.abs(np.array(f[:]) - want).max() <= 2e-2 + 2e-4 * np.abs(want).max(), (sd, f[:], want)
             assert np.array_equal(want, est[38 + 19 * sd:41 + 19 * sd])        # the archive reports the same vector for toe and heel
             checked += 1
-    if os.path.exists(O.lib_path(ref=True)):   # closed loop against the live archive
-        o = O.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'), ref=True)
-        Lr = O.load(ref=True)
-        Lr.o_state_output_step.argtypes = [C.c_void_p, C.c_void_p]
-        y, y2, co = pkg.state_out_t(), pkg.state_out_t(), (C.c_char * 1336)()
-        u = O.make_pd(pTarget=PD_TARGET, pGain=PD_PGAIN, dGain=PD_DGAIN)
-        big = 0.0
-        for k in range(800):
-            o.step_pd(u, y, co)
-            Lr.o_state_output_step(C.byref(co), C.byref(y2))
-            for name in ('leftFoot', 'rightFoot'):
-                for fld in ('toeForce', 'heelForce'):
-                    a, b = field(y, name + '.' + fld), field(y2, name + '.' + fld)
-                    assert np.abs(a - b).max() <= 2e-2 + 2e-4 * np.abs(a).max(), (k, name, fld, a, b)
-                    big = max(big, np.abs(a).max())
-        assert big > 30                                       # standing: the springs carry the weight
-        checked += 1
+    V = archive_runs()                                  # closed loop: the archive's records every 50 ticks of the fixed-PD run
+    L.o_state_output_step.argtypes = [C.c_void_p, C.c_void_p]
+    big = 0.0
+    for co, ya in zip(V['pd_cassie_out'], V['pd_state_out']):
+        y, y2 = pkg.state_out_t.from_buffer_copy(ya.tobytes()), pkg.state_out_t()
+        L.o_state_output_step((C.c_char * 1336).from_buffer_copy(co.tobytes()), C.byref(y2))
+        for name in ('leftFoot', 'rightFoot'):
+            for fld in ('toeForce', 'heelForce'):
+                a, b = field(y, name + '.' + fld), field(y2, name + '.' + fld)
+                assert np.abs(a - b).max() <= 2e-2 + 2e-4 * np.abs(a).max(), (name, fld, a, b)
+                big = max(big, np.abs(a).max())
+    assert big > 30                                           # standing: the springs carry the weight
+    checked += 1
     assert checked > 0

@@ -1,12 +1,11 @@
 """The estimator's filters (pelvis.position / translationalVelocity / externalForce, terrain.height of state_out_t; SURVEY.md 8f-1).
-Three implementations are compared: the reference's closed block (live when /root/reference is present, else its committed outputs
-tests/golden/estimator_sequence.npz), the oracle's restatement (oracle/cassie_oracle.c o_est_filter_step) and the product's host object
+Three implementations are compared: the reference's closed block (its committed outputs tests/golden/estimator_sequence.npz and
+archive_runs.npz), the oracle's restatement (oracle/cassie_oracle.c o_est_filter_step) and the product's host object
 (csrc/estimator_host.h EstimatorFilter through cassie_b200_estimator_filter_step).  No GPU involved."""
 import ctypes as C
 import os
 
 import numpy as np
-import pytest
 
 from conftest import GOLDEN, PD_DGAIN, PD_PGAIN, PD_TARGET
 
@@ -107,33 +106,34 @@ def test_product_filter_equals_oracle_filter_on_random_sequences(oracle_mod, pkg
 
 
 def test_oracle_estimator_against_live_archive_in_closed_loop(oracle_mod, pkg):
-    """the whole restated estimator (stateless part + filters) beside the closed block in a closed-loop run; the filters alone, fed the block's own
-    stateless outputs, to rounding.  End to end the leg forces limit the agreement (the block evaluates them in single precision)."""
-    if not os.path.exists(oracle_mod.lib_path(ref=True)):
-        pytest.skip('reference archive not built here')
+    """the whole restated estimator (stateless part + filters) in a closed-loop run of 1200 calls beside the closed block's outputs on the same run
+    (tests/golden/archive_runs.npz, every 50th call); the filters alone, fed the block's own stateless outputs (its 400-call sequence), to
+    rounding.  End to end the leg forces limit the agreement (the block evaluates them in single precision)."""
     O = oracle_mod
-    L = O.load(ref=True)
+    L = O.load()
     L.o_est_new.restype = C.c_void_p
     L.o_est_free.argtypes = [C.c_void_p]
     L.o_est_filter_step.argtypes = [C.c_void_p, C.c_void_p]
     L.o_state_output_step_full.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-    o = O.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'), ref=True)
+    V, S = np.load(os.path.join(GOLDEN, 'archive_runs.npz')), np.load(os.path.join(GOLDEN, 'estimator_sequence.npz'))
+    o = O.OracleSim(os.path.join(GOLDEN, 'cassie.omodel'))
     u = O.make_pd(pTarget=PD_TARGET, pGain=PD_PGAIN, dGain=PD_DGAIN)
     y, y3, y4, co = pkg.state_out_t(), pkg.state_out_t(), pkg.state_out_t(), (C.c_char * 1336)()
     e1, e2 = L.o_est_new(), L.o_est_new()
     err_filter, err_full = 0.0, 0.0
-    for k in range(1200):
-        o.step_pd(u, y, co)                                   # y: the archive's state_out_t for this call
-        C.memmove(C.byref(y3), C.byref(y), C.sizeof(y))
-        for i in range(3):
-            y3.pelvis.position[i] = y3.pelvis.translationalVelocity[i] = y3.pelvis.externalForce[i] = 0
-        y3.terrain.height = 0
+    for x, want in zip(S['stateless'], S['filtered']):
+        _load_stateless(y3, x)
         L.o_est_filter_step(e1, C.byref(y3))
-        L.o_state_output_step_full(e2, C.byref(co), C.byref(y4))
-        want = _filtered(y)
         err_filter = max(err_filter, _rel(_filtered(y3), want).max())
-        err_full = max(err_full, _rel(_filtered(y4), want).max())
-        assert not any(y.pelvis.externalMoment[:]) and not any(y.terrain.slope[:])     # never written by the block
+    ticks = list(V['pd_tick'])
+    for k in range(ticks[-1] + 1):
+        o.step_pd(u, y, co)
+        L.o_state_output_step_full(e2, C.byref(co), C.byref(y4))
+        if k in ticks:
+            ya = pkg.state_out_t.from_buffer_copy(V['pd_state_out'][ticks.index(k)].tobytes())     # the archive's state_out_t for this call
+            want = _filtered(ya)
+            err_full = max(err_full, _rel(_filtered(y4), want).max())
+            assert not any(ya.pelvis.externalMoment[:]) and not any(ya.terrain.slope[:])     # never written by the block
     L.o_est_free(e1)
     L.o_est_free(e2)
     assert abs(want[8]) > 1 and abs(want[2]) > 0.3
